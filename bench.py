@@ -9,6 +9,12 @@ synthetic CSR of BASELINE.json configs[1]: ALS d=128 on 10M x 1M, 1B nnz (SURVEY
 `value` = nnz * steps / device time with everything resident in HBM; `e2e` = the same iteration driven
 through the reference-facing host-pointer C ABI (bfl_als_partial_update: pinned-host CSR chunks H2D,
 updated factor rows D2H inside the timed region).  One JSON line on stdout (rank 0).
+
+`--dump-outputs DIR` writes, after the timed steps, the factor matrices the last timed step left behind as
+DIR/<name>.npy (see dump_outputs); the workload and the initial factors are seeded, so two builds run with the same
+arguments can be compared output for output.  Rows of more than 1536 nonzeros are summed chunk by chunk with float
+atomics, so two runs of one build already differ: on C2 with --warmup 3 --steps 3 by up to 2.3e-3 of the largest
+entry of P and of Q (one B200, 1000 W power limit).
 """
 import argparse
 import json
@@ -22,6 +28,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: nothing is cached next to the sources
 
 WORKLOADS = {
     # name: users, items, nnz, d, mean degree generator
@@ -186,6 +193,24 @@ def init_factors_t(rows, d, device, seed):
     g.manual_seed(seed)
     # abs(N(0, 1/d^2)) (buffalo/algo/als.py:85-86)
     return torch.abs(torch.randn(rows, d, device=device, generator=g, dtype=torch.float32) * (1.0 / d ** 2)).contiguous()
+
+
+DUMP_BYTES_PER_ARRAY = 16 << 20  # at most four arrays per path: 64 MB in all
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Writes each output matrix as <out_dir>/<name>.npy (float32): all of it when it fits in DUMP_BYTES_PER_ARRAY,
+    else a sample of its rows, the same sorted rows on every run (np.random.default_rng(seed), drawn in dict order)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(seed)
+    for name, F in arrays.items():
+        rows = F.shape[0]
+        n = min(rows, DUMP_BYTES_PER_ARRAY // (4 * F[0].numel()))
+        if n < rows:
+            F = F[torch.from_numpy(np.sort(rng.choice(rows, size=n, replace=False))).to(F.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), F.float().cpu().numpy())
+    log("wrote %s to %s" % (", ".join(k + ".npy" for k in arrays), out_dir))
 
 
 def algorithmic_bytes(nnz, rows, d):
@@ -366,7 +391,13 @@ def main():
     ap.add_argument("--tc-min-class", type=int, default=None, help="first row-length class solved by the tensor-core kernel (default: library's)")
     ap.add_argument("--exchange", default=os.environ.get("BFL_EXCHANGE", "p2p"), choices=["p2p", "allgather"],
                     help="multi-GPU: fused peer stores from the solve kernel (default) or an NCCL all-gather per half-epoch")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the factors of the last step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     if args.algo != "als":
         sys.path.insert(0, os.path.join(ROOT, "benchmarks"))
         import sgd_bench
@@ -462,6 +493,8 @@ def main():
     launches = _cabi.lib().bfl_kernel_launch_count() - launches0
     ms = t0e.elapsed_time(t1e)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"P": P, "Q": Q})   # every rank holds the full factors after the exchange
     if world > 1:
         t = torch.tensor([ms], device=device, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -144,6 +144,8 @@ def main(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     drv.finalize()
+    if args.dump_outputs and rank == 0:
+        bench.dump_outputs(args.dump_outputs, dict(P=P, Q=Q, Qb=Qb) if algo == "bpr" else dict(P=P, Q=Q))
     mean_trials = None
     if trials is not None:
         tt = trials.to(torch.float32)

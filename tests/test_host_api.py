@@ -349,3 +349,21 @@ def test_bench_zipf_generator_chunked_equals_unchunked():
             ref = (ri.copy(), rk.copy(), ck.copy())
         else:
             assert (ref[0] == ri).all() and (ref[1] == rk).all() and (ref[2] == ck).all()
+
+
+def test_bench_dump_outputs_is_a_fixed_bounded_sample(tmp_path):
+    """bench.py --dump-outputs: a matrix larger than the per-array budget is cut to the same sorted row sample on every
+    run, a small one is written whole, always as float32, and four arrays stay within 64 MB."""
+    import torch
+    import bench
+    P = torch.arange(300000 * 16, dtype=torch.float32).reshape(300000, 16)     # row r holds 16 r .. 16 r + 15
+    Qb = torch.arange(50, dtype=torch.float64).reshape(50, 1)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"P": P, "Qb": Qb})
+    a, b = np.load(tmp_path / "a" / "P.npy"), np.load(tmp_path / "b" / "P.npy")
+    assert a.dtype == np.float32 and a.shape[1] == 16 and 0 < a.shape[0] < 300000
+    assert 4 * a.nbytes <= 64 << 20 and np.array_equal(a, b)
+    rows = a[:, 0] / 16
+    assert (np.diff(rows) > 0).all() and np.array_equal(a, P.numpy()[rows.astype(np.int64)])
+    qb = np.load(tmp_path / "a" / "Qb.npy")
+    assert qb.dtype == np.float32 and np.array_equal(qb, Qb.numpy())
